@@ -7,7 +7,8 @@ sign + projector + one Qwen3-14B block pass) -> tokenizer decode, for ``--bs`` i
   python bench.py --gpus N --steps K --warmup W            # this repo (one process per GPU under torchrun for N > 1)
   python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host CPU cores (oracle port)
 
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0). ``--dump-outputs DIR`` also writes what the last timed step returned (rank 0) as
+``DIR/<name>.npy``; the weights, prompt and sampler noise are seeded, so the same arguments give the same inputs.
 """
 from __future__ import annotations
 
@@ -26,12 +27,37 @@ MODEL = "BitDance-14B-64x"
 METRIC = "1024px images/sec (14B-64x)"
 P_LLM, P_HEAD, P_COND, P_PROJ = 13.2125e9, 1.7585e9, 26.2e6, 26.4e6   # SURVEY.md §8d
 KV_BYTES_PER_TOKEN = 163840
+DUMP_BYTES = 64 << 20        # --dump-outputs: at most this many bytes in all (arrays, indices, headers, outputs.json)
 DEFAULT_LLM_STREAM = True    # one persistent launch per Qwen3 AR block (on par with the chained kernels: profiles/r02_bench_*)
 
 
 def algorithmic_bytes_per_ar_step(R: int, S: int, avg_ctx: float) -> float:
     """SURVEY.md §8(d): weights streamed once per AR step (cond+uncond batched, cond_embed hoisted) + KV reads."""
     return 2 * P_LLM + (S + 1) * 2 * (P_HEAD - P_COND) + 2 * (P_COND + P_PROJ) + R * avg_ctx * KV_BYTES_PER_TOKEN
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as ``out_dir/<name>.npy`` in float32 and their shapes to ``out_dir/outputs.json``. When they would
+    exceed DUMP_BYTES, each is replaced by the same fixed, seeded sample of its C-order flattened elements (a share of the
+    budget proportional to its size), and the flat indices kept go to ``out_dir/<name>.index.npy`` (float64, exact
+    integers): 12 bytes per kept element."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    n = sum(a.size for a in arrays.values())
+    room = DUMP_BYTES - (1 << 16)                 # .npy headers and outputs.json
+    sampled = 4 * n > room
+    os.makedirs(out_dir, exist_ok=True)
+    manifest = {}
+    for name, a in arrays.items():
+        manifest[name] = {"shape": list(a.shape), "sampled": sampled}
+        if sampled:
+            keep = int(a.size * (room // 12) // n)
+            idx = np.sort(np.random.default_rng(0).choice(a.size, size=keep, replace=False))
+            np.save(os.path.join(out_dir, name + ".index.npy"), idx.astype(np.float64))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+    with open(os.path.join(out_dir, "outputs.json"), "w") as f:
+        json.dump(manifest, f)
 
 
 class ClockSampler:
@@ -293,7 +319,11 @@ def main():
     ap.add_argument("--graph", type=int, default=1, help="replay the AR step as a CUDA graph (1) or launch it eagerly (0)")
     ap.add_argument("--llm-stream", type=int, default=-1,
                     help="Qwen3 AR block as one persistent launch (1) or as chained kernels (0); -1: BD_LLM_STREAM or the default")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the tokens and image of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -380,8 +410,8 @@ def main():
         tokens, packed = eng.gen_tokens(ce, ue, se, h=h, w=w, num_images=B, guidance_scale=args.guidance,
                                         num_sampling_steps=S, num_steps=args.ar_steps)
         if args.ar_steps is not None:
-            return None
-        return eng.decode(tokens, h, w)
+            return tokens, None
+        return tokens, eng.decode(tokens, h, w)
 
     # ---- the PUBLIC call: BitDanceT2IPipeline.generate(prompt, ...) -> list[PIL.Image] (t2i_pipeline.py:110-155) over the
     # same engine: host tokenizer, embedding lookup, token ids H2D, the whole path, uint8 pixels D2H, PIL conversion
@@ -415,6 +445,7 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    torch.manual_seed(1234 + rank)    # the sampler noise: the same for every run with the same arguments
     for _ in range(args.warmup):
         gen_resident(ids_dev)
     barrier()
@@ -423,11 +454,18 @@ def main():
     with ClockSampler(local) as clk:
         barrier()
         ev0.record()
-        for _ in range(args.steps):
-            gen_resident(ids_dev)
+        for i in range(args.steps):
+            if i < args.steps - 1:
+                gen_resident(ids_dev)
+            else:                             # only the final step's outputs are kept (for --dump-outputs)
+                last = gen_resident(ids_dev)
         ev1.record()
         barrier()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        tokens, image = last
+        dump_outputs(args.dump_outputs, {"tokens": tokens} if image is None else {"tokens": tokens, "image": image})
+    del last
     launches = lib.bd_launch_count() - launches0
     # per-phase split of the last configuration (one extra, untimed-for-the-metric pass)
     eng.gen_tokens(embed[ids_dev[:64]], embed[ids_dev[64:67]], embed[ids_dev[67:]], h=h, w=w, num_images=B,

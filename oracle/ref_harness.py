@@ -31,6 +31,24 @@ def _eager_flash(q, k, v, causal=False):
     return (a @ vh).transpose(1, 2).contiguous()
 
 
+def shim_transformers():
+    """Shims B and C, once: what the reference's calls into transformers need (also for driving Qwen3 directly)."""
+    from transformers import DynamicCache
+    from transformers.modeling_utils import ALL_ATTENTION_FUNCTIONS
+
+    if not hasattr(DynamicCache, "_bd_shim"):
+        DynamicCache.__getitem__ = lambda s, i: (s.layers[i].keys, s.layers[i].values)
+        DynamicCache._bd_shim = True
+        _orig = ALL_ATTENTION_FUNCTIONS["sdpa"]
+
+        def _sdpa(module, q, k, v, attention_mask=None, **kw):
+            if attention_mask is not None and attention_mask.dim() == 4:
+                attention_mask = attention_mask[..., : k.shape[-2]]
+            return _orig(module, q, k, v, attention_mask=attention_mask, **kw)
+
+        ALL_ATTENTION_FUNCTIONS["sdpa"] = _sdpa
+
+
 _done = False
 _ns = None
 
@@ -96,20 +114,7 @@ def import_reference():
         return _eager_flash(q, k, v, causal=bool(kw.get("causal", a[2] if len(a) > 2 else False)))
 
     fh.flash_attn_func = _flash
-    from transformers import DynamicCache
-    from transformers.modeling_utils import ALL_ATTENTION_FUNCTIONS
-
-    if not hasattr(DynamicCache, "_bd_shim"):
-        DynamicCache.__getitem__ = lambda s, i: (s.layers[i].keys, s.layers[i].values)
-        DynamicCache._bd_shim = True
-        _orig = ALL_ATTENTION_FUNCTIONS["sdpa"]
-
-        def _sdpa(module, q, k, v, attention_mask=None, **kw):
-            if attention_mask is not None and attention_mask.dim() == 4:
-                attention_mask = attention_mask[..., : k.shape[-2]]
-            return _orig(module, q, k, v, attention_mask=attention_mask, **kw)
-
-        ALL_ATTENTION_FUNCTIONS["sdpa"] = _sdpa
+    shim_transformers()
     _done = True
     _ns = types.SimpleNamespace(fh=fh, sx=sx, ae=ae, mu=mu, t2i=t2i)
     return _ns

@@ -1,7 +1,7 @@
 """``bench.py --impl reference`` (the driver's reference arm) on the "tiny" configuration: runs the UNMODIFIED reference's
 ``gen_image`` on the host cores, prints ONE JSON line with the contract keys, and bounds its sample (calibration step +
 deadline: the host arm runs in a killable subprocess and the number is derived from whatever finished) whatever
---steps / --warmup are passed. Needs the reference (dev container, or oracle/_ref on the GPU box)."""
+--steps / --warmup are passed. The tests that run the arm need the reference (oracle/ref_harness.py); the others do not."""
 import json
 import os
 import subprocess
@@ -10,7 +10,6 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.reference
 
 
 def run(*extra):
@@ -23,6 +22,7 @@ def run(*extra):
     return json.loads(lines[0])
 
 
+@pytest.mark.reference
 def test_reference_arm_line():
     line = run("--steps", "2", "--warmup", "1")
     assert "unavailable" not in line, line
@@ -34,6 +34,7 @@ def test_reference_arm_line():
     assert line["config"]["ar_steps_run"] == {"warmup": 1, "timed": 2}
 
 
+@pytest.mark.reference
 def test_reference_arm_deadline_is_reported_not_fatal():
     env = dict(os.environ, CUDA_VISIBLE_DEVICES="", BD_REF_DEADLINE_S="1")
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--model", "tiny"],

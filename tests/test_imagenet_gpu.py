@@ -1,6 +1,6 @@
 """The ImageNet class-conditional generator on the GPU (bitdance_b200/imagenet.py; SURVEY.md section 8 rows a16 / f1)
-against the CPU oracle (oracle/imagenet.py, autocast-bf16 policy) and — when the shipped copy of the reference is
-present (oracle/make_ref.py) — against the UNMODIFIED ``BitDance.sample`` running on the same GPU under CUDA autocast."""
+against the CPU oracle (oracle/imagenet.py, autocast-bf16 policy) and against what the UNMODIFIED ``BitDance.sample``
+returned on a B200 under CUDA autocast (tests/golden/reference_gpu_pins.npz)."""
 import pytest
 import torch
 
@@ -136,73 +136,34 @@ def test_imagenet_api_mirror_and_reference_on_gpu():
 
 
 def test_imagenet_vs_unmodified_reference_on_gpu():
-    from oracle import ref_harness as rh
-    if not rh.available():
-        pytest.skip("reference copy not shipped (oracle/make_ref.py)")
-    import sys
-    import torch._dynamo
-    import torch.nn as nn
-    for k in [k for k in sys.modules if k == "src" or k.startswith("src.")]:
-        del sys.modules[k]
-    sys.path.insert(0, rh.REF + "/imagenet_gen")
-    old = torch._dynamo.config.disable
-    torch._dynamo.config.disable = True
-    try:
-        from src import model_parallel as mp
-        assert mp.__file__.startswith(rh.REF)
-
-        class _VaeStub(nn.Module):
-            def __init__(self, *a, **k):
-                super().__init__()
-
-            def decode(self, x):
-                return x
-
-        real = mp.VQModel
-        mp.VQModel = _VaeStub
-        cfg = dict(CFG)
-        try:
-            ref = mp.BitDance(dim=128, n_layer=2, n_head=2, diff_layers=2, diff_dim=128, diff_adanln_layers=1, latent_dim=32,
-                              down_size=16, patch_size=1, resolution=64, diff_batch_mul=1, cls_token_num=4, num_classes=10,
-                              parallel_num=4, parallel_mode="patch").eval()
-        finally:
-            mp.VQModel = real
-        from bitdance_b200.imagenet import ImageNetEngine, imagenet_spec
-        from bitdance_b200.synth import synth_state_dict
-        sd = synth_state_dict(imagenet_spec(cfg), seed=4, std=0.08)
-        missing = ref.load_state_dict(sd, strict=False)
-        assert not missing.unexpected_keys and all(k.startswith("vae.") for k in missing.missing_keys)
-        ref = ref.cuda()
-        eng = ImageNetEngine(sd, cfg, ae=None)
-        S, cfg_scale = 4, 3.0
-        class_ids = torch.tensor([3, 7, 1]).cuda()
-        # same noise for both: record the reference's randn draws (generation order) and replay them in the engine
-        rec = []
-        o1, o2 = torch.randn, torch.randn_like
-        torch.randn = lambda *a, **k: (rec.append(o1(*a, **k)) or rec[-1])
-        torch.randn_like = lambda a, **k: (rec.append(o2(a, **k)) or rec[-1])
-        try:
-            torch.manual_seed(11)
-            with torch.no_grad(), torch.amp.autocast("cuda", dtype=torch.bfloat16):
-                grid_ref = ref.sample(class_ids, S, cfg_scale=cfg_scale, cfg_schedule="linear")
-        finally:
-            torch.randn, torch.randn_like = o1, o2
-        steps = eng.h * eng.w // eng.pn
-        assert len(rec) == steps * (S + 1)
-        noise = [torch.stack(rec[i * (S + 1):(i + 1) * (S + 1)]).float().contiguous() for i in range(steps)]
-        tokens, _ = eng.sample_tokens(class_ids, S, cfg_scale, noise=noise)
-        grid = eng.tokens_to_grid(tokens)
-        pn = eng.pn
-        ref_tok = grid_ref.float()
-        a_all = (grid == ref_tok).float().mean().item()
-        # first block = the first p x p patch of the grid
-        p = eng.ps
-        a0 = (grid[:, :, :p, :p] == ref_tok[:, :, :p, :p]).float().mean().item()
-        print(f"ImageNet vs the unmodified reference on this GPU (CUDA autocast): first-block token agreement {a0:.4f}, "
-              f"whole grid {a_all:.4f}")
-        assert a0 > 0.95 and a_all > 0.65
-    finally:
-        torch._dynamo.config.disable = old
-        sys.path.remove(rh.REF + "/imagenet_gen")
-        for k in [k for k in sys.modules if k == "src" or k.startswith("src.")]:
-            del sys.modules[k]
+    """Against the UNMODIFIED ``BitDance.sample`` run on a B200 under CUDA autocast with the same weights (the seeded
+    synth_state_dict below): its token grid and the noise it drew are stored in tests/golden/reference_gpu_pins.npz
+    (tests/golden/make_reference_gpu_pins.py), and the noise is replayed in the engine."""
+    import os
+    import numpy as np
+    from bitdance_b200.imagenet import ImageNetEngine, imagenet_spec
+    from bitdance_b200.synth import synth_state_dict
+    golden = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_gpu_pins.npz"))
+    cfg = dict(CFG)
+    sd = synth_state_dict(imagenet_spec(cfg), seed=4, std=0.08)
+    eng = ImageNetEngine(sd, cfg, ae=None)
+    S, cfg_scale = 4, 3.0
+    class_ids = torch.tensor([3, 7, 1]).cuda()
+    flat, rec, o = torch.from_numpy(golden["imagenet_noise"]), [], 0
+    for shape in golden["imagenet_noise_shapes"]:
+        n = int(np.prod(shape))
+        rec.append(flat[o:o + n].view(*(int(d) for d in shape)).cuda())
+        o += n
+    steps = eng.h * eng.w // eng.pn
+    assert len(rec) == steps * (S + 1)
+    noise = [torch.stack(rec[i * (S + 1):(i + 1) * (S + 1)]).float().contiguous() for i in range(steps)]
+    tokens, _ = eng.sample_tokens(class_ids, S, cfg_scale, noise=noise)
+    grid = eng.tokens_to_grid(tokens)
+    ref_tok = torch.from_numpy(golden["imagenet_grid"]).float().to(grid.device)
+    a_all = (grid == ref_tok).float().mean().item()
+    # first block = the first p x p patch of the grid
+    p = eng.ps
+    a0 = (grid[:, :, :p, :p] == ref_tok[:, :, :p, :p]).float().mean().item()
+    print(f"ImageNet vs the unmodified reference on a B200 (CUDA autocast): first-block token agreement {a0:.4f}, "
+          f"whole grid {a_all:.4f}")
+    assert a0 > 0.95 and a_all > 0.65

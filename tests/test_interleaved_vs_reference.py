@@ -1,24 +1,27 @@
 """Interleaved text+image inference against the UNMODIFIED reference ``MLLModel.forward_inference_block_causal``
-(modeling/mllm.py:696-897), on CPU in fp32 with the tiny random model (dev container only: the reference's ``mllm.py``
-imports its ``data`` package, which is not shipped to the GPU box).
+(modeling/mllm.py:696-897), on CPU in fp32 with the tiny model of ``bitdance_b200.synthetic.tiny_state_dicts()``.
 
-What can be pinned and is:
-  * plan [user text, model image] == the reference's own ``gen_image(cond, remove_first_user_block(cond))`` bit for bit — the
+What can be pinned and is, against the reference's outputs stored in tests/golden/reference_pins.npz
+(tests/golden/make_reference_pins.py; the sampler noise is drawn again here from the same seeds):
+  * plan [user text, model image] == ``oracle/pipeline.py::gen_image(cond, remove_first_user_block(cond))`` — the
     equivalence the mirror's image item rests on (it hands the accumulated context to the same block generator);
   * plan [user text, user image, model image] (editing) == ``oracle/pipeline.py::gen_image`` fed with the context the MIRROR's
-    bookkeeping builds (start tokens + encode_image + <|vision_end|> in BOTH streams, unconditional text =
-    remove_first_user_block): pins that bookkeeping against the reference's.
+    bookkeeping builds (start tokens + the reference's encode_image of the source + <|vision_end|> in BOTH streams,
+    unconditional text = remove_first_user_block): pins that bookkeeping against the reference's.
 What cannot: the reference's TEXT branch raises — without a cache at mllm.py:798 (``past_key_values[0][0]`` of None), after a
 generated image on the second token (a 2-D ``(1, hidden)`` tensor fed back as ``inputs_embeds``, :857 -> rotary shape
-error). Both are asserted here, as the evidence for DESIGN.md section 2c's "text loop parity-unpinned"."""
+error). Both are asserted by the last test, which runs the reference itself and needs its whole source tree (its
+``mllm.py`` imports the reference's ``data`` package), as the evidence for DESIGN.md section 2c's "text loop parity-unpinned"."""
+import os
+
+import numpy as np
 import pytest
 import torch
 from torch import nn
 
-pytestmark = pytest.mark.reference
-
 TEXT = "<|im_start|>user\na photo of the red cat<|im_end|>\n<|im_start|>assistant\n"
 U, M_ = {"from": "user"}, {"from": "model"}
+S, GUIDANCE, PN = 3, 3.0, 16
 
 
 class _Cfg(dict):
@@ -26,12 +29,82 @@ class _Cfg(dict):
 
 
 @pytest.fixture(scope="module")
+def golden():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_pins.npz"))
+
+
+@pytest.fixture(scope="module")
+def tiny():
+    """the weights and tokenizer of the stored reference runs"""
+    from bitdance_b200.synthetic import MODELS, synthetic_tokenizer, tiny_state_dicts
+    sds = tiny_state_dicts()
+    tok, _ = synthetic_tokenizer(512, PN)
+    cfg = {k: v for k, v in MODELS["tiny"]["llm"].items() if k != "vocab_size"}
+    return sds, tok, cfg
+
+
+def _noise(shapes):
+    """the reference's draws in the stored run, in order, from the same global-RNG state; grouped per AR step"""
+    rec = [torch.randn(tuple(int(d) for d in s)) for s in shapes]
+    steps = 64 // PN
+    assert len(rec) == steps * (S + 1)
+    return [rec[i * (S + 1):(i + 1) * (S + 1)] for i in range(steps)]
+
+
+def _oracle_image(tiny, cond, uncond, noise):
+    from oracle import pipeline as op
+    sds, tok, cfg = tiny
+    ids = lambda ts: [tok.convert_tokens_to_ids(t) for t in ts]
+    start = ids(["<|vision_start|>", "<|res_8|>", "<|res_8|>"] + [f"<|query_{i}|>" for i in range(1, PN)])
+    with torch.no_grad():
+        _, img = op.gen_image(sd_llm=sds["llm"], cfg_llm=cfg, embed=sds["llm"]["model.embed_tokens.weight"],
+                              sd_head=sds["head"], sd_proj=sds["proj"], sd_ae=sds["ae"], cond_ids=None, uncond_ids=None,
+                              cond_emb=cond, uncond_emb=uncond, start_ids=start, h=8, w=8, pn=PN, num_images=1,
+                              guidance=GUIDANCE, S=S, noise=noise, head_dim=128)
+    return img
+
+
+def test_reference_t2i_plan_is_gen_image(golden, tiny):
+    from bitdance_b200.modeling.utils import remove_first_user_block
+    sds, tok, _ = tiny
+    embed = sds["llm"]["model.embed_tokens.weight"]
+    E = lambda s: embed[torch.tensor(tok.encode(s))]
+    torch.manual_seed(5)
+    noise = _noise(golden["interleaved_t2i_noise_shapes"])
+    img = _oracle_image(tiny, E(TEXT), E(remove_first_user_block(TEXT)), noise)
+    img_ref = torch.from_numpy(golden["interleaved_t2i_image"])
+    assert img.shape == img_ref.shape == (1, 3, 32, 32)
+    err = (img - img_ref).abs().max().item()
+    assert err < 1e-3 * max(1.0, img_ref.abs().max().item()), err
+
+
+def test_reference_editing_plan_vs_oracle_with_mirror_bookkeeping(golden, tiny):
+    from bitdance_b200.modeling.utils import remove_first_user_block
+    sds, tok, _ = tiny
+    torch.manual_seed(7)
+    noise = _noise(golden["interleaved_edit_noise_shapes"])
+    # the context as bitdance_b200/modeling/mllm.py builds it, around the reference's encode_image of the source image
+    embed = sds["llm"]["model.embed_tokens.weight"]
+    E = lambda ids: embed[torch.tensor(list(ids))]
+    start3 = [tok.convert_tokens_to_ids(t) for t in ("<|vision_start|>", "<|res_8|>", "<|res_8|>")]
+    pre = torch.from_numpy(golden["interleaved_edit_source_latent"])
+    assert pre.shape == (64, 256)
+    end = E([tok.convert_tokens_to_ids("<|vision_end|>")])
+    cond = torch.cat([E(tok.encode(TEXT)), E(start3), pre, end])
+    uncond = torch.cat([E(tok.encode(remove_first_user_block(TEXT))), E(start3), pre, end])
+    img = _oracle_image(tiny, cond, uncond, noise)
+    img_ref = torch.from_numpy(golden["interleaved_edit_image"])
+    assert img.shape == img_ref.shape == (1, 3, 32, 32)
+    err = (img - img_ref).abs().max().item()
+    assert err < 1e-3 * max(1.0, img_ref.abs().max().item()), err
+
+
+@pytest.fixture(scope="module")
 def world():
-    import os
-    if not os.path.isdir("/root/reference/data"):
-        pytest.skip("needs the full reference checkout (modeling/mllm.py imports data.data_utils)")
-    from bitdance_b200.synthetic import synthetic_tokenizer
     from oracle import ref_harness as rh
+    if not os.path.isdir(os.path.join(rh.REF, "data")):
+        pytest.skip("runs the reference itself: needs its whole source tree (modeling/mllm.py imports data.data_utils)")
+    from bitdance_b200.synthetic import synthetic_tokenizer
     from oracle import ref_runner as rr
     rh.import_reference()
     mllm = rh.import_reference_mllm()
@@ -60,81 +133,7 @@ def world():
     return m, pipe, tok
 
 
-def _capture_noise(fn):
-    rec = []
-    o1, o2 = torch.randn, torch.randn_like
-
-    def r1(*a, **k):
-        t = o1(*a, **k)
-        rec.append(t.clone())
-        return t
-
-    def r2(a, **k):
-        t = o2(a, **k)
-        rec.append(t.clone())
-        return t
-
-    torch.randn, torch.randn_like = r1, r2
-    try:
-        out = fn()
-    finally:
-        torch.randn, torch.randn_like = o1, o2
-    return out, rec
-
-
-def test_reference_t2i_plan_is_gen_image(world):
-    from bitdance_b200.modeling.utils import remove_first_user_block
-    m, pipe, tok = world
-    kw = dict(max_length_vision=64, sample_steps=3, image_size=[32, 32], cfg_scale=3.0)
-    with torch.no_grad():
-        torch.manual_seed(5)
-        out = m.forward_inference_block_causal([dict(type="text", **U), dict(type="image", **M_)], [TEXT], [], **kw)
-        torch.manual_seed(5)
-        ref = pipe.gen_image(TEXT, remove_first_user_block(TEXT), guidance_scale=3.0, num_sampling_steps=3, max_length=64,
-                             num_images=1, image_size=[32, 32])
-    img = out["generated_image"][0]
-    assert out["generated_text"] == [] and img.shape == (1, 3, 32, 32) and torch.equal(img, ref)
-
-
-def test_reference_editing_plan_vs_oracle_with_mirror_bookkeeping(world):
-    from bitdance_b200.modeling.utils import remove_first_user_block
-    from oracle import pipeline as op
-    from oracle import ref_runner as rr
-    m, pipe, tok = world
-    S, guidance, pn = 3, 3.0, 16
-    src = torch.rand(1, 3, 32, 32, generator=torch.Generator().manual_seed(1)) * 2 - 1
-    plan = [dict(type="text", **U), dict(type="image", **U), dict(type="image", **M_)]
-    with torch.no_grad():
-        torch.manual_seed(7)
-        out, noise = _capture_noise(lambda: m.forward_inference_block_causal(
-            plan, [TEXT], [src.clone()], max_length_vision=64, sample_steps=S, image_size=[32, 32], cfg_scale=guidance))
-        img_ref = out["generated_image"][0]
-        steps = 64 // pn
-        assert len(noise) == steps * (S + 1)
-        per_step = [noise[i * (S + 1):(i + 1) * (S + 1)] for i in range(steps)]
-        # the context as bitdance_b200/modeling/mllm.py builds it
-        embed = m.llm_model.model.embed_tokens.weight.detach().float()
-        E = lambda ids: embed[torch.tensor(list(ids))]
-        start3 = [tok.start_of_image_id, tok.res_8_id, tok.res_8_id]
-        pre = m.encode_image([src.clone()])[0].float()
-        assert pre.shape == (64, 256)
-        end = E([tok.end_of_image_id])
-        cond = torch.cat([E(tok.encode(TEXT)), E(start3), pre, end])
-        uncond = torch.cat([E(tok.encode(remove_first_user_block(TEXT))), E(start3), pre, end])
-        start = start3 + [getattr(tok, f"query_{i}_id") for i in range(1, pn)]
-        c = rr.CONFIGS["tiny"]["llm"]
-        cfg = {k: v for k, v in c.items() if k != "vocab_size"}
-        f32 = lambda sd: {k: v.detach().float() for k, v in sd.items()}
-        tokens, img = op.gen_image(sd_llm=f32(m.llm_model.state_dict()), cfg_llm=cfg, embed=embed,
-                                   sd_head=f32(pipe.vision_head.state_dict()), sd_proj=f32(pipe.embed_vision_mlp.state_dict()),
-                                   sd_ae=f32(pipe.ae.state_dict()), cond_ids=None, uncond_ids=None, cond_emb=cond,
-                                   uncond_emb=uncond, start_ids=start, h=8, w=8, pn=pn, num_images=1, guidance=guidance, S=S,
-                                   noise=per_step, head_dim=128)
-    assert img.shape == img_ref.shape == (1, 3, 32, 32)
-    err = (img - img_ref).abs().max().item()
-    assert err < 1e-3 * max(1.0, img_ref.abs().max().item()), err
-
-
+@pytest.mark.reference
 def test_reference_text_branch_raises(world):
     m, pipe, tok = world
     with torch.no_grad():
